@@ -3,6 +3,7 @@
 ([256, T=1000, V=29] per GPU, beam 100, cutoff_top_n 40, cutoff_prob 1.0, no LM; synthetic CTC-like input).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+                    [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK / LOCAL_RANK / WORLD_SIZE); utterances are independent, so each
 rank decodes its own [256, T, V] shard and there is no data-path collective ("weak" scaling, N=8 is
@@ -222,6 +223,9 @@ def bench_lm(args, cfg, config, rank, world, local_rank, dev, K, W, cores):
         return
     val = B * world * K / float(t[0])
     top1 = "".join(L29[x] for x in out[0][0, 0, :out[3][0, 0]])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tokens=out[0].numpy(), timesteps=out[2].numpy(), scores=out[1].numpy(),
+                     lens=out[3].numpy(), n_results=dec.last_n_results.numpy(), flags=dec.last_flags.numpy())
     line = {"metric": METRIC, "value": val, "unit": "utterances/s", "n_gpus": world, "steps": K, "warmup": W,
             "ms_per_step": 1e3 * float(t[0]) / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "f32", "data": "synthetic", "config": config,
@@ -248,6 +252,8 @@ def main():
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-strong", action="store_true", help="skip the fixed-2048 (BASELINE config 3) leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     rank = int(os.environ.get("RANK", "0"))
@@ -326,12 +332,14 @@ def main():
         sampler.start()  # (before the warm-up: a 10-step timed region is only ~50 ms, a sample every 100 ms)
     m = measure(lib, dev, local_rank, cfg, B, rank, K, W, barrier)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, **{k: v.cpu().numpy() for k, v in m["device"].items()})
     # BASELINE config 3 beside it (SURVEY.md 8e): a FIXED total of 2048 utterances split over the ranks, so that the
     # driver's N = 1, 2, 4, 8 runs carry the strong-scaling curve next to the weak one
     strong = None
     if args.config == "c2" and not args.no_strong:
         c3 = CONFIGS["c3"]
-        strong = measure(lib, dev, local_rank, c3, c3["B"] // world, 1000 + rank, min(K, 5), 3, barrier)
+        strong = measure(lib, dev, local_rank, c3, c3["B"] // world, 1000 + rank, K, 3, barrier)
 
     # ---- reduce over ranks (max time) ----------------------------------------------------------------------------
     vals = [m["total_ms"], m["e2e_ms"], float(m["n_err"]), float(m["n_tie"]), 0.0 if m["same"] else 1.0]
@@ -388,7 +396,7 @@ def main():
     }
     if strong:
         gb = CONFIGS["c3"]["B"] // world * world
-        ks = min(K, 5)
+        ks = K
         line["strong_c3"] = {
             "workload": CONFIGS["c3"]["name"], "global_batch": gb, "batch_per_gpu": gb // world, "steps": ks,
             "value": gb * ks / (float(t[5]) / 1e3), "unit": "utterances/s", "ms_per_step": float(t[5]) / ks,
@@ -489,8 +497,30 @@ def measure(lib, dev, local_rank, cfg, B, seed, K, W, barrier):
     same = bool(torch.equal(h_sc, d_sc.cpu()) and torch.equal(h_len, d_len.cpu()))
     return dict(total_ms=total_ms, e2e_ms=e2e_s * 1e3, kern_ms=kern_ms, n_err=n_err, n_tie=n_tie, same=same, h2d=h2d,
                 d2h=d2h, probs_cpu=probs_cpu,
+                device=dict(tokens=d_tok, timesteps=d_ts, scores=d_sc, lens=d_len, n_results=d_nres, flags=d_flags),
                 host=dict(tokens=h_tok.numpy(), timesteps=h_ts.numpy(), scores=h_sc.numpy(), lens=h_len.numpy(),
                           n_results=h_nres.numpy(), ties=h_flags.numpy()))
+
+
+def dump_outputs(directory, tokens, timesteps, scores, lens, n_results, flags):
+    """Writes the results of the last timed step as float32 DIR/<name>.npy, so that two builds can be compared output
+    for output (the inputs are seeded): scores, lens, n_results and flags of every utterance, and tokens / timesteps of
+    a fixed, seeded sample of utterances (sample_utterances) that keeps the files under ~50 MB in all.  Rows past an
+    utterance's n_results and steps past a beam's length hold no result: they are written as 0 and -1."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    B, beam, T = tokens.shape
+    n_results = n_results.astype(np.int64)
+    row = np.arange(beam)[None, :] < n_results[:, None]
+    lens = np.where(row, lens, 0)
+    k = max(1, min(B, (48 << 20) // (beam * T * 8)))
+    idx = np.sort(np.random.default_rng(0).choice(B, k, replace=False))
+    step = np.arange(T)[None, None, :] < lens[idx][:, :, None]
+    out = {"scores": np.where(row, scores, 0.0), "lens": lens, "n_results": n_results, "flags": flags,
+           "sample_utterances": idx, "tokens": np.where(step, tokens[idx], -1),
+           "timesteps": np.where(step, timesteps[idx], -1)}
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), np.asarray(a, np.float32))
 
 
 def cpu_legs(m, cfg, cores):

@@ -148,6 +148,11 @@ double ref_scorer_sent_from_labels(void *scorer, const int *labels, int n) {
   return s->get_sent_log_prob(s->split_labels(v));
 }
 
+// Scorer::get_log_cond_prob(words) for one n-gram (scorer.cpp:74-93): what tests/golden/make_lm_tables.py records
+double ref_scorer_cond_from_words(void *scorer, const char *const *words, int n) {
+  return static_cast<Scorer *>(scorer)->get_log_cond_prob(std::vector<std::string>(words, words + n));
+}
+
 // The language model's vocabulary as KenLM enumerates it (what Scorer::load_lm collects, scorer.cpp:55-72),
 // '\n'-separated into buf; returns the number of bytes needed.
 size_t ref_lm_vocabulary(const char *lm_path, char *buf, size_t cap) {

@@ -66,8 +66,23 @@ def emit_lm(name, probs, alpha, beta, seq_lens=None, **kw):
     print(name, probs.shape, "n_results", r["n_results"][:4], "top-1", top[:3])
 
 
+def emit_ref_build_cases():
+    """recorded/ref_build_cases.npz: the reference's outputs for tests/test_oracle.py REF_BUILD_CASES (inputs from seeds)"""
+    from tests.test_oracle import REF_BUILD_CASES, ref_build_inputs
+    arrays = {}
+    for i, cfg in enumerate(REF_BUILD_CASES):
+        probs, V, kw = ref_build_inputs(cfg)
+        r = Reference([str(v) for v in range(V)]).decode(probs, **kw)
+        L = max(1, int(r["lens"].max()))
+        r["tokens"], r["timesteps"] = r["tokens"][:, :, :L], r["timesteps"][:, :, :L]
+        arrays.update({"case%d/%s" % (i, k): v for k, v in r.items()})
+    os.makedirs(os.path.join(HERE, "recorded"), exist_ok=True)
+    np.savez_compressed(os.path.join(HERE, "recorded", "ref_build_cases.npz"), **arrays)
+
+
 if __name__ == "__main__":
     from ctcdecode_b200.synth import text_probs
+    emit_ref_build_cases()
     texts = ["the cat sat on the mat", "a dog ran fast", "the dog sat on a mat the cat ran"]
     emit_lm("lm_tiny_a15_b08_beam32", text_probs(texts, L29, 160, seed=1).numpy(), 1.5, 0.8, beam=32)
     emit_lm("lm_tiny_a0_b0_beam20", text_probs(texts[:2], L29, 120, seed=2).numpy(), 0.0, 0.0, beam=20)

@@ -24,6 +24,12 @@ def load_lm(name):
     return probs, seq_lens, kw, ref, float(z["lm"][0]), float(z["lm"][1])
 
 
+def recorded_ref_build(i):
+    """The reference build's outputs for tests/test_oracle.py REF_BUILD_CASES[i] (tests/golden/make_golden.py)."""
+    z = np.load(os.path.join(HERE, "recorded", "ref_build_cases.npz"))
+    return {f.split("/", 1)[1]: z[f] for f in z.files if f.startswith("case%d/" % i)}
+
+
 def load(name):
     z = np.load(os.path.join(HERE, name + ".npz"))
     beam, top_n, blank, log_input = [int(x) for x in z["params"]]

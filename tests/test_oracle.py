@@ -1,7 +1,7 @@
 """The oracle is pinned before it is trusted: the plain-C restatement (oracle/ctc_oracle.c) must reproduce
 (1) the reference's own known answers (reference tests/test_decode.py:13-32,37-91),
 (2) the committed outputs of the unmodified reference build (tests/golden, all beams / timesteps / scores),
-(3) the reference build itself on fresh seeded inputs whenever oracle/_ref is present."""
+(3) the reference build's recorded outputs on seeded inputs, and the build itself whenever oracle/_ref is present."""
 import numpy as np
 import pytest
 
@@ -43,21 +43,32 @@ def test_cport_matches_reference_golden(cport, name):
         assert skipped == 0
 
 
-@pytest.mark.skipif(not orc.reference_available(), reason="oracle/_ref not built (needs /root/reference)")
-@pytest.mark.parametrize("cfg", [
+REF_BUILD_CASES = [
     dict(B=3, T=150, V=29, seed=11, beam=48),
     dict(B=2, T=90, V=40, seed=12, beam=24, cutoff_top_n=12),
     dict(B=2, T=60, V=300, seed=13, beam=40, cutoff_prob=0.99),
     dict(B=2, T=80, V=29, seed=14, beam=30, cutoff_prob=0.5),
     dict(B=4, T=100, V=29, seed=15, beam=50, flat=True),
-])
-def test_cport_matches_reference_build(cport, cfg):
+]
+
+
+def ref_build_inputs(cfg):
+    """-> probs, V, decoder keywords"""
     cfg = dict(cfg)
     B, T, V, seed = cfg.pop("B"), cfg.pop("T"), cfg.pop("V"), cfg.pop("seed")
     probs = (flat_probs(B, T, V, seed) if cfg.pop("flat", False) else ctc_like_probs(B, T, V, seed)).numpy()
-    ref = orc.Reference([str(i) for i in range(V)]).decode(probs, **cfg)
-    got = cport.decode(probs, **cfg)
-    compare(ref, got, got["ties"], str(cfg))
+    return probs, V, cfg
+
+
+@pytest.mark.parametrize("cfg", REF_BUILD_CASES)
+def test_cport_matches_reference_build(cport, cfg):
+    """against the reference build's recorded outputs for these inputs (tests/golden/make_golden.py), and against the
+    build itself when oracle/_ref is present"""
+    probs, V, kw = ref_build_inputs(cfg)
+    got = cport.decode(probs, **kw)
+    compare(golden_util.recorded_ref_build(REF_BUILD_CASES.index(cfg)), got, got["ties"], str(cfg))
+    if orc.reference_available():
+        compare(orc.Reference([str(i) for i in range(V)]).decode(probs, **kw), got, got["ties"], str(cfg) + " (live)")
 
 
 def test_cport_streaming_equals_offline(cport):
